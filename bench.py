@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the DistEGNN hot path on B200 (contract: see the task statement / DESIGN.md §Measurement).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload synth1m]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload synth1m] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one complete FastEGNN forward (4 layers, all virtual-node all-reduces) over the WHOLE graph
@@ -24,6 +24,9 @@ metric = graph-steps/s (BASELINE.json), `edges_per_sec` = Σ_p E_p × graph-step
 --impl reference times ONLY the CPU path, at FULL size: the whole 1M-node graph (N>1: the block-diagonal union of the
 N partitions, identical arithmetic to N-rank DistEGNN — BASELINE.md §3), 1 warm-up + as many timed forwards as fit
 --ref-budget-s; `steps` reports how many were timed.
+
+--dump-outputs DIR writes what the last timed step returned, node_loc.npy [N, 3] and virtual_loc.npy [B, 3, C]; inputs
+and weights are generated from fixed seeds, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -38,6 +41,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 from distegnn_b200 import synth  # noqa: E402
@@ -66,7 +70,30 @@ def parse():
     ap.add_argument("--ref-budget-s", type=float, default=420.0,
                     help="--impl reference: wall-clock budget for full-size CPU forwards (1 warm-up + timed steps)")
     ap.add_argument("--no-dist-parity", action="store_true", help="skip the multi-GPU parity cases before the timed region")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps write the outputs of the last one as DIR/<name>.npy (float32; with N>1 "
+                         "ranks one file per rank), for comparing two builds on the same seeded inputs")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
+
+
+DUMP_MAX_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(d: str, outputs, rank: int, world: int) -> None:
+    """Write each output as DIR/<name>.npy in float32 (DIR/<name>.rank<r>.npy with N>1 ranks).  If the outputs exceed
+    DUMP_MAX_BYTES in all, each keeps a seeded sample of its rows (in order), the same from run to run."""
+    os.makedirs(d, exist_ok=True)
+    total = world * sum(t.numel() * 4 for t in outputs.values())
+    for name, t in outputs.items():
+        t = t.detach().float().cpu()
+        if total > DUMP_MAX_BYTES:
+            keep = max(1, t.shape[0] * DUMP_MAX_BYTES // total)
+            rows = torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(rank))[:keep].sort().values
+            t = t[rows]
+        np.save(os.path.join(d, name + ("" if world == 1 else f".rank{rank}") + ".npy"), t.numpy())
 
 
 def peaks():
@@ -266,8 +293,10 @@ def run_reference(args, w, rank, world):
         if times and (time.perf_counter() - t0) + max(times) > args.ref_budget_s:
             break
         t1 = time.perf_counter()
-        fn(inp)
+        out, X = fn(inp)
         times.append(time.perf_counter() - t1)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"node_loc": out, "virtual_loc": X}, rank, 1)
     t_step = sum(times) / len(times)
     value = 1.0 / t_step
     line = {
@@ -416,6 +445,8 @@ def run_ours(args, w, rank, world, local_rank):
         wall = time.perf_counter() - wall0
         launches = be.launches - launches0
         clocks = sampler.stop()
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"node_loc": out, "virtual_loc": X}, rank, world)
         t_dev = sum(s.elapsed_time(e) for s, e in evs) * 1e-3
         model._timing = None
         model.cuda_graph = False                          # e2e below uses fresh device tensors every step

@@ -30,6 +30,10 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 REF = "/root/reference"
 OUT = os.path.join(ROOT, "tests", "golden")
+INIT_SEED = 0                       # torch.manual_seed before the reference constructor
+if ROOT not in sys.path:
+    sys.path.insert(0, ROOT)
+from tests.helpers import MAX_FIXTURE_BYTES, tensor_digest  # noqa: E402
 
 
 def import_reference():
@@ -108,7 +112,7 @@ def _to_np(d):
 
 
 def run_reference(FastEGNN, kw, inp, scale, dtype, world_size=1):
-    torch.manual_seed(0)
+    torch.manual_seed(INIT_SEED)
     model = FastEGNN(hidden_nf=64, world_size=world_size, **kw)
     sd = model.state_dict()
     for k in sd:
@@ -162,7 +166,16 @@ def main():
             for i, t in enumerate(tr[key]):
                 blob[f"trace.{key}.{i}"] = t.numpy()
         blob["meta.kw"] = np.array(repr(kw))
-        np.savez_compressed(os.path.join(OUT, name + ".npz"), **blob)
+        path = os.path.join(OUT, name + ".npz")
+        np.savez_compressed(path, **blob)
+        if os.path.getsize(path) > MAX_FIXTURE_BYTES:
+            # untouched init too large to store: keep its seed and a digest per tensor instead; tests.helpers.load_golden
+            # regenerates the weights and checks them against the digests
+            assert scale == 1.0, name
+            blob = {k: v for k, v in blob.items() if not k.startswith("sd.")}
+            blob["meta.seed"] = np.array(INIT_SEED)
+            blob.update({"sdsha." + k: np.array(tensor_digest(v)) for k, v in sd.items()})
+            np.savez_compressed(path, **blob)
         print(name, "N", inp["node_feat"].shape[0], "E", inp["edge_index"].shape[1],
               "max|out32-out64|", float((out32.double() - out64).abs().max()))
 

@@ -27,13 +27,32 @@ ROOT = os.path.dirname(HERE)
 sys.path.insert(0, ROOT)
 sys.path.insert(0, HERE)
 from make_golden import OUT, import_reference  # noqa: E402
-from tests.helpers import DIST_CASE, SINGLE_CASES, golden_inputs, load_golden  # noqa: E402
+from tests.helpers import DIST_CASE, MAX_FIXTURE_BYTES, SINGLE_CASES, golden_inputs, load_golden  # noqa: E402
+
+GRAD_SAMPLE = 1536      # entries kept of each large gradient when the whole fixture would exceed MAX_FIXTURE_BYTES
 
 
 def cotangents(seed, n, B, C, dtype):
     g = torch.Generator().manual_seed(seed)
     return torch.randn(n, 3, generator=g, dtype=torch.float64).to(dtype), \
         torch.randn(B, 3, C, generator=g, dtype=torch.float64).to(dtype)
+
+
+def sample_large_grads(blob, seed=0):
+    """Each nonzero gradient of more than GRAD_SAMPLE entries -> a seeded sample of its flat entries ("grad.<k>") that
+    includes the entry of largest magnitude, plus their sorted flat indices ("idx.grad.<k>"; tests.helpers.grad_sample).
+    All-zero gradients stay whole: they compress to nothing and the tests check them entry by entry."""
+    rng = np.random.default_rng(seed)
+    out = {}
+    for k, v in blob.items():
+        flat = v.reshape(-1)
+        if k.startswith("grad.") and flat.size > GRAD_SAMPLE and np.abs(flat).max() > 0:
+            idx = np.unique(np.append(rng.choice(flat.size, GRAD_SAMPLE - 1, replace=False), np.abs(flat).argmax()))
+            out["idx." + k] = idx.astype(np.int32)
+            out[k] = flat[idx]
+        else:
+            out[k] = v
+    return out
 
 
 def reference_grads(FastEGNN, kw, sd, inp, cot_out, cot_X, dtype, world_size=1):
@@ -76,7 +95,10 @@ def main():
         g32, _ = reference_grads(FastEGNN, kw, sd, inp, cot_out.float(), cot_X.float(), torch.float32)
         blob = {"grad." + k: v.numpy() for k, v in grads.items()}
         blob.update({"cot.out": cot_out.numpy(), "cot.X": cot_X.numpy(), "loss": np.array(loss)})
-        np.savez_compressed(os.path.join(OUT, name + ".grads.npz"), **blob)
+        path = os.path.join(OUT, name + ".grads.npz")
+        np.savez_compressed(path, **blob)
+        if os.path.getsize(path) > MAX_FIXTURE_BYTES:
+            np.savez_compressed(path, **sample_large_grads(blob))
         worst = max(float((g32[k].double() - grads[k]).abs().max() / grads[k].abs().max().clamp(min=1e-30)) for k in grads)
         print(name, "loss", loss, "params", len(grads), "max rel |grad32 - grad64| over parameters", worst)
 
